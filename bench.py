@@ -7,6 +7,7 @@ Float32 DArray of N * 2^30 elements, one 2^30-element (4 GiB) localpart per GPU 
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--log2n 30]            # our arm (one process per GPU under torchrun)
   python bench.py --impl reference ...                                         # the reference's CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                                       # also write the last timed step's y (sampled) and sum(y)
 
 Prints ONE JSON line (rank 0).  value = whole-job algorithmic GB/s with inputs resident in HBM; e2e = same metric through the
 public API with HOST (pinned) input each step; roofline = the dominant kernel (the broadcast) against the measured HBM peak;
@@ -113,8 +114,7 @@ def cpu_leg(log2n_per_worker, steps, warmup, workers=None):
     remotecall / serialisation overhead is NOT reproduced (that flatters the reference)."""
     from oracle import core as ocore
 
-    ocore.build()
-    cores = ocore.num_procs()
+    cores = ocore.num_procs()          # loads the liboracle_core.so that build() made; never recompiles into the tree
     n_per = 1 << log2n_per_worker
     tried = {}
     if workers:
@@ -273,11 +273,44 @@ def parity_halo(dab, rt, dst, seed, rows_total, r0, c0):
     return {"ok": bad_all == 0, "columns_per_rank": len(cols), "mismatching_columns": bad_all, "tol": "bit-exact"}
 
 
+DUMP_ELEMS = 1 << 22    # y values written by --dump-outputs over all ranks: 16 MiB of Float32
+
+
+def dump_offsets(n_per, world):
+    """Start offsets (within a localpart) of the WINDOW-element windows of y that --dump-outputs writes; None: the whole localpart."""
+    import numpy as np
+
+    per_rank = DUMP_ELEMS // world
+    if n_per <= per_rank:
+        return None
+    return np.sort(np.random.default_rng(SEED + 5).choice(n_per // WINDOW, per_rank // WINDOW, replace=False)) * WINDOW
+
+
+def dump_outputs(dab, rt, y, s, n_per, world, out_dir):
+    """What the timed step hands its caller, written after its last step: ``y.npy`` (Float32; the whole of y when it holds at most
+    DUMP_ELEMS elements, else the windows of every localpart at dump_offsets(), concatenated in rank order) and ``sum.npy`` (the
+    Float32 sum(y)).  Same arguments -> same inputs and same sample, so two builds can be compared file by file."""
+    import numpy as np
+
+    ch = dab.localpart(y)
+    offs = dump_offsets(n_per, world)
+    if offs is None:
+        part = ch.to_numpy().reshape(-1)
+    else:
+        part = np.concatenate([_d2h_window(dab, rt, ch, int(off), WINDOW) for off in offs])
+    parts = rt.allgather_object(part)
+    if rt.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "y.npy"), np.concatenate(parts).astype(np.float32))
+        np.save(os.path.join(out_dir, "sum.npy"), np.array([s], dtype=np.float32))
+
+
 
 def main():
+    sys.dont_write_bytecode = True     # the benchmark leaves the tree as build() left it (no __pycache__ of the modules it imports)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--log2n", type=int, default=30, help="log2 of the elements per GPU (default 2^30 = 4 GiB chunk)")
@@ -285,7 +318,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (y, sum(y)) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     warmup = max(3, args.warmup)
@@ -366,6 +402,8 @@ def main():
     l0 = rt.launches()
     ms, s = timed(step, args.steps)
     launches = rt.launches() - l0
+    if args.dump_outputs:
+        dump_outputs(dab, rt, y, s, n_per, world, args.dump_outputs)
     ms = max_over_ranks(ms)
     value = 12.0 * N * args.steps / (ms * 1e-3) / 1e9
 

@@ -408,6 +408,40 @@ def test_bench_host_logic_against_the_host_memory_abi():
     assert line["n_gpus"] == 1 and line["steps"] == 2 and line["e2e"]["h2d_bytes_per_step"] == 4 * (1 << 16) and line["gpu_launches"] > 0
 
 
+@pytest.mark.parametrize("log2n", [16, 23])
+def test_bench_dump_outputs_against_the_host_memory_abi(tmp_path, log2n):
+    """``bench.py --dump-outputs DIR`` (C ABI emulated over host memory): y.npy holds y = fl(fl(a*x)+b) bit-exact -- all of it at 2^16
+    elements, the seeded windows at 2^23 -- sum.npy the printed sum, and a second run with the same arguments writes the same files."""
+    import importlib.util
+    import json
+    import subprocess
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = 1 << log2n
+    dumps = []
+    for run in ("a", "b"):
+        out = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "run_on_hostmem.py"), "bench.py", "--log2n", str(log2n), "--steps", "1",
+                            "--warmup", "3", "--no-cpu", "--no-extras", "--no-parity", "--dump-outputs", str(out)],
+                           cwd=ROOT, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, (r.stdout + r.stderr)[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert sorted(p.name for p in out.iterdir()) == ["sum.npy", "y.npy"]
+        y, s = np.load(out / "y.npy"), np.load(out / "sum.npy")
+        assert y.dtype == np.float32 and s.dtype == np.float32 and s.shape == (1,) and float(s[0]) == line["sum"]
+        assert y.nbytes + s.nbytes <= 64 << 20
+        offs = bench.dump_offsets(n, 1)
+        if offs is None:
+            want = ocore.affine_f32(ocore.rand_u01_f32(bench.SEED, 0, n), bench.A_COEF, bench.B_COEF)
+        else:
+            assert y.size == bench.DUMP_ELEMS < n
+            want = np.concatenate([ocore.affine_f32(ocore.rand_u01_f32(bench.SEED, int(o), bench.WINDOW), bench.A_COEF, bench.B_COEF) for o in offs])
+        assert np.array_equal(y.view(np.uint32), want.view(np.uint32))
+        dumps.append((y, s))
+    assert all(np.array_equal(u.view(np.uint32), v.view(np.uint32)) for u, v in zip(*dumps))
+
+
 def test_smoke_host_logic_against_the_host_memory_abi():
     """``__graft_entry__.smoke()`` (what the driver runs on the B200 before the bench) with the C ABI emulated over host memory: its host side
     -- layouts vs the oracle, map!, broadcast, sum / maximum, sum(dims=1), the halo read, A*B, the strided view, sort -- runs through."""

@@ -13,16 +13,14 @@
   * ``norm(x, p)`` for p = 0, -Inf and general p (host-side compositions of the fused map + reduce);
   * general broadcasts over more than 4 dimensions (``collapse_dims`` in ``_broadcast.py``; reference src/broadcast.jl is N-d).
 
-STATUS: these tests have NOT been executed on hardware yet.  What is verified on CPU: the sort-by-key composition (key|position words,
-two rounds for 64-bit keys, gather) step by step in ``tests/hostmem_abi.py`` against a stable ``isless`` argsort, the whole host flow
-of ``_sort.py`` against the oracle (``tests/test_cpu_sort.py``), and that the collapsed box of ``collapse_dims`` addresses exactly the
-elements NumPy's broadcasting reads (``tests/test_cpu_host.py``), that the Int128 reduce kernels compile with NVRTC for sm_100a and
-that the host side (slot decoding, wrap-around fold) is exact (``tests/test_cpu_jit_reduce.py``).  What only a B200 can verify: the two small sort-by-key kernels,
-their ctypes bindings, and the N-d broadcast through the real NVRTC kernel.  The module therefore runs LAST (file name) and is marked
-``xfail(strict=False)``: a pass is reported as XPASS, a failure cannot hide a regression elsewhere or turn the tier red for code that
-was never claimed as measured.  Order inside the module: host-side compositions of GPU-tested kernels first, new NVRTC device code
-(extension prelude, Int128 carriers) next, the two new hand-written kernels (sort by key) last -- a fault in newer code cannot take the
-evidence for the rest with it.  ``pytest tests/test_gpu_zz_last_session.py -m gpu --runxfail`` shows real failures as failures."""
+Also verified on CPU: the sort-by-key composition (key|position words, two rounds for 64-bit keys, gather) step by step in
+``tests/hostmem_abi.py`` against a stable ``isless`` argsort, the whole host flow of ``_sort.py`` against the oracle
+(``tests/test_cpu_sort.py``), and that the collapsed box of ``collapse_dims`` addresses exactly the elements NumPy's broadcasting reads
+(``tests/test_cpu_host.py``), that the Int128 reduce kernels compile with NVRTC for sm_100a and that the host side (slot decoding,
+wrap-around fold) is exact (``tests/test_cpu_jit_reduce.py``).  What only a B200 can verify: the two small sort-by-key kernels, their
+ctypes bindings, and the N-d broadcast through the real NVRTC kernel.  The module runs LAST (file name), and inside it host-side
+compositions of GPU-tested kernels come first, new NVRTC device code (extension prelude, Int128 carriers) next, the two hand-written
+sort-by-key kernels last -- a fault in newer code cannot take the evidence for the rest with it."""
 import ctypes as C
 
 import numpy as np
@@ -33,8 +31,7 @@ from oracle import darray_oracle as orc
 INT128_BIG_N = (1 << 22) + 5                    # the CPU dry run of these tests (tests/test_cpu_host.py) shrinks the big sizes
 SORT_BY_KEY_SIZES = (1, 2, 33, 1024, 1025, 4097, 100003, (1 << 20) + 17)
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.xfail(strict=False, reason="added in the last session of round 2, never executed on a GPU (budget spent)")]
+pytestmark = pytest.mark.gpu
 
 
 def test_broadcast_more_than_4_dims(dab, rt8):
