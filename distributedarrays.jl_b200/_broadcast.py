@@ -490,8 +490,8 @@ def run_local(rt, expr: Expr, out: B200Array, largs: List[LocalArg]):
             if ab is not None:
                 a = np.asarray(ab[0], dtype=out.dtype)
                 b = np.asarray(ab[1], dtype=out.dtype)
-                _lib.call("dab_affine", ctx, code, C.c_void_p(out.ptr), C.c_void_p(x0.arr.ptr), C.c_void_p(a.ctypes.data),
-                          C.c_void_p(b.ctypes.data), n)
+                # deferred: a reduction of `out` issued next runs fused with it (runtime.Runtime.defer_affine); any other call launches it
+                rt.defer_affine(code, out.ptr, x0.arr.ptr, a, b, n)
                 rt.last_kernel = "dab_affine"
                 return
             if expr.op in _UN and _is_arg(expr.args[0], 0):

@@ -89,6 +89,7 @@ _SIGS = {
     "dab_jit_compile_check_reduce": (_i32, [C.c_char_p, _i32, _i32, _i32, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_sz)]),
     "dab_reduce": (_i32, [_vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "dab_reduce_host": (_i32, [_vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "dab_affine_reduce": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "dab_reduce_result_dtype": (_i32, [_i32, _i32, _i32, C.POINTER(_i32)]),
     "dab_combine_ordered": (_i32, [_i32, _i32, _vp, _sz, _vp]),
     "dab_reducedim": (_i32, [_vp, _i32, _i32, _i32, _vp, _sz, _sz, _sz, _vp, _i32]),
@@ -111,6 +112,7 @@ _SIGS = {
     "dab_send": (_i32, [_vp, _vp, _sz, _i32]),
     "dab_recv": (_i32, [_vp, _vp, _sz, _i32]),
     "dab_mapreduce_all": (_i32, [_vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "dab_affine_mapreduce_all": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "dab_mailbox_create": (_i32, [_vp, _vp]),
     "dab_mailbox_attach": (_i32, [_vp, _vp, _i32, _i32]),
     "dab_mailbox_detach": (_i32, [_vp]),
@@ -157,8 +159,33 @@ def check(status: int, ctx=None) -> None:
     raise _EXC.get(status, DabError)(status, text)
 
 
+# Contexts that hold a deferred launch (``Runtime.defer_affine``), keyed by the context's address.  Every C-ABI call on such a context
+# launches the deferred op first, so the stream sees the calls in the order they were made.
+_DEFERRED = {}
+
+
+def ctx_key(ctx):
+    return ctx.value if isinstance(ctx, C.c_void_p) else ctx
+
+
+FUSED_STEP = ("dab_affine_reduce", "dab_affine_mapreduce_all")
+
+
+def serves_fused_step() -> bool:
+    """Whether the loaded binding has the fused broadcast + reduce entry points.  libdab200.so always has them (``lib()`` refuses a
+    library that lacks a declared symbol); a stand-in object that implements only the unfused C ABI does not, and the runtime then
+    launches every broadcast at once instead of deferring it."""
+    L = lib()
+    return all(hasattr(L, name) for name in FUSED_STEP)
+
+
 def call(name: str, ctx, *args):
-    """Call ``name(ctx, *args)`` and raise on a non-zero status."""
+    """Call ``name(ctx, *args)`` and raise on a non-zero status.  A launch deferred on ``ctx`` is made first; an error it returns is
+    raised here."""
+    if _DEFERRED:
+        owner = _DEFERRED.get(ctx_key(ctx))
+        if owner is not None:
+            owner.flush()
     check(getattr(lib(), name)(ctx, *args), ctx)
 
 

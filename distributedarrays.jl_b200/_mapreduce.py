@@ -219,6 +219,9 @@ def _mapreduce_expr(expr: Expr, opc: int, d: DArray, others: Sequence, return_pa
     return (res, vals) if return_partials else res
 
 
+_FUSED_OPS = (_lib.SUM, _lib.PROD, _lib.MAX, _lib.MIN)    # the reductions dab_affine_reduce serves
+
+
 def _mapreduce_all(f, op, d: DArray, return_partials: bool = False, others: Sequence = ()):
     opc = op if isinstance(op, int) else _op_code(op)
     if others:
@@ -231,14 +234,42 @@ def _mapreduce_all(f, op, d: DArray, return_partials: bool = False, others: Sequ
     rt = d.rt
     pp = C.c_void_p(param.ctypes.data) if param is not None else None
     rdt = _result_dtype(d.dtype, opc, mapc)
+    code = dab_dtype(d.dtype)
+    fusable = mapc == _lib.MAP_ID and opc in _FUSED_OPS and code in (_lib.F32, _lib.F64) and rt.pending is not None
+
+    def take_pending(ch):
+        """The deferred ``y .= a.*x .+ b`` when it writes exactly this chunk: the reduce then runs fused with it."""
+        return rt.take_pending(code, ch.ptr, ch.size) if fusable else None
+
     if rt.workers_per_rank == 1 and d.layout.pids == rt.workers() and not return_partials:
         # production mapping, one chunk per GPU: reduce kernel + cross-worker combine + ordered fold in ONE C-ABI call
         ch = d.chunks[rt.myid()]
         out = np.zeros(2, dtype=np.uint64)
-        _lib.call("dab_mapreduce_all", rt.ctx, dab_dtype(d.dtype), opc, mapc, pp, C.c_void_p(ch.ptr), ch.size, C.c_void_p(out.ctypes.data))
+        p = take_pending(ch)
+        if p is not None:
+            _lib.call("dab_affine_mapreduce_all", rt.ctx, code, C.c_void_p(p.y), C.c_void_p(p.x), C.c_void_p(p.a.ctypes.data),
+                      C.c_void_p(p.b.ctypes.data), p.n, opc, C.c_void_p(out.ctypes.data))
+        else:
+            _lib.call("dab_mapreduce_all", rt.ctx, code, opc, mapc, pp, C.c_void_p(ch.ptr), ch.size, C.c_void_p(out.ctypes.data))
         return out.view(np.uint8)[:rdt.itemsize].view(rdt)[0]
-    code = dab_dtype(d.dtype)
-    host = _gather_slots(d, lambda pid, ch, slot: _lib.call("dab_reduce", rt.ctx, code, opc, mapc, pp, C.c_void_p(ch.ptr), ch.size, C.c_void_p(slot)))
+    # the deferred broadcast can only have written one local chunk: take it out now (the slot allocation below is a C-ABI call, which
+    # would launch it) and run that chunk's reduce fused with it.  The reduces of the other chunks neither read nor write its x or y.
+    p = next((q for q in map(take_pending, d.chunks.values()) if q is not None), None) if fusable else None
+
+    def launch(pid, ch, slot):
+        nonlocal p
+        if p is not None and (p.y, p.n) == (ch.ptr, ch.size):
+            q, p = p, None
+            _lib.call("dab_affine_reduce", rt.ctx, code, C.c_void_p(q.y), C.c_void_p(q.x), C.c_void_p(q.a.ctypes.data),
+                      C.c_void_p(q.b.ctypes.data), q.n, opc, C.c_void_p(slot))
+        else:
+            _lib.call("dab_reduce", rt.ctx, code, opc, mapc, pp, C.c_void_p(ch.ptr), ch.size, C.c_void_p(slot))
+
+    try:
+        host = _gather_slots(d, launch)
+    finally:
+        if p is not None:                                   # not reached (an error came first): it stays the pending op
+            rt.defer_affine(p.dtype, p.y, p.x, p.a, p.b, p.n)
     res, vals = _fold(host, d.layout.pids, rdt, opc)
     return (res, vals) if return_partials else res
 

@@ -234,20 +234,18 @@ int32_t dab_recv(dab_ctx* ctx, void* recv_dev, size_t nbytes, int32_t peer) {
     return DAB_OK;
 }
 
-// Base._mapreduce(f, op, ::IndexCartesian, d::DArray), reference src/mapreduce.jl:29-35, for ONE chunk per rank:
-//   results = asyncmap(procs(d)) do p; remotecall_fetch(mapreduce(f, op, localpart(d))) end     -> kernel + allgather
-//   reduce(op, results)                                                                        -> ordered left fold
-int32_t dab_mapreduce_all(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const void* map_param, const void* x, size_t n,
-                          void* out_host) {
-    DAB_ENTER(ctx);
-    DAB_REQUIRE(ctx, out_host, DAB_ERR_ARG, "dab_mapreduce_all: null out");
-    int32_t rdt;
-    if (op == DAB_EXTREMA) return dab_fail(ctx, DAB_ERR_UNSUPPORTED, "dab_mapreduce_all: extrema combines through dab_reduce + dab_allgather");
-    if (dab_reduce_result_dtype(dtype, op, map, &rdt) != DAB_OK) return dab_fail(ctx, DAB_ERR_ARG, "bad dtype/op");
+}  // extern "C"
+
+namespace {
+
+// The combine of dab_mapreduce_all around one chunk reduce: `launch(slot)` enqueues the kernel that writes this rank's 16-byte result
+// slot (dab_reduce, or dab_affine_reduce for the fused broadcast + sum).  rdt: the result dtype.
+template <typename Launch>
+int32_t mapreduce_all_combine(dab_ctx* ctx, int32_t op, int32_t rdt, size_t n, void* out_host, Launch launch) {
     if ((ctx->mbox_ranks > 1 || !ctx->comm || ctx->nranks == 1) && n > 0) {
         // fused path: ONE kernel = chunk reduce + peer-memory all-gather + ordered fold + scalar into pinned host memory
         ctx->fuse_op = op;
-        int32_t st = dab_reduce(ctx, dtype, op, map, map_param, x, n, ctx->result_slot);
+        int32_t st = launch(ctx->result_slot);
         ctx->fuse_op = -1;
         if (st != DAB_OK) return st;
         DAB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -258,7 +256,7 @@ int32_t dab_mapreduce_all(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, 
         memcpy(out_host, &bits, dab_dtype_size(rdt));
         return DAB_OK;
     }
-    int32_t st = dab_reduce(ctx, dtype, op, map, map_param, x, n, ctx->result_slot);
+    int32_t st = launch(ctx->result_slot);
     if (st != DAB_OK) return st;
     const int P = ctx->comm ? ctx->nranks : 1;
     const void* src = ctx->result_slot;
@@ -279,6 +277,38 @@ int32_t dab_mapreduce_all(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, 
     memset(out_host, 0, 8);
     memcpy(out_host, res, es);
     return DAB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+// Base._mapreduce(f, op, ::IndexCartesian, d::DArray), reference src/mapreduce.jl:29-35, for ONE chunk per rank:
+//   results = asyncmap(procs(d)) do p; remotecall_fetch(mapreduce(f, op, localpart(d))) end     -> kernel + allgather
+//   reduce(op, results)                                                                        -> ordered left fold
+int32_t dab_mapreduce_all(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const void* map_param, const void* x, size_t n,
+                          void* out_host) {
+    DAB_ENTER(ctx);
+    DAB_REQUIRE(ctx, out_host, DAB_ERR_ARG, "dab_mapreduce_all: null out");
+    int32_t rdt;
+    if (op == DAB_EXTREMA) return dab_fail(ctx, DAB_ERR_UNSUPPORTED, "dab_mapreduce_all: extrema combines through dab_reduce + dab_allgather");
+    if (dab_reduce_result_dtype(dtype, op, map, &rdt) != DAB_OK) return dab_fail(ctx, DAB_ERR_ARG, "bad dtype/op");
+    return mapreduce_all_combine(ctx, op, rdt, n, out_host,
+                                 [&](void* slot) { return dab_reduce(ctx, dtype, op, map, map_param, x, n, slot); });
+}
+
+// y .= a.*x .+ b then sum(y) (any of SUM PROD MAX MIN) of one chunk per rank: dab_mapreduce_all with dab_affine_reduce as the chunk
+// reduce, so the step reads x, writes y and never reads y back when the kernel fuses.
+int32_t dab_affine_mapreduce_all(dab_ctx* ctx, int32_t dtype, void* y, const void* x, const void* a, const void* b, size_t n, int32_t op,
+                                 void* out_host) {
+    DAB_ENTER(ctx);
+    DAB_REQUIRE(ctx, ((x && y) || n == 0) && a && b, DAB_ERR_ARG, "dab_affine: null pointer");
+    DAB_REQUIRE(ctx, out_host, DAB_ERR_ARG, "dab_mapreduce_all: null out");
+    int32_t rdt;
+    if (op == DAB_EXTREMA) return dab_fail(ctx, DAB_ERR_UNSUPPORTED, "dab_mapreduce_all: extrema combines through dab_reduce + dab_allgather");
+    if (dab_reduce_result_dtype(dtype, op, DAB_MAP_ID, &rdt) != DAB_OK) return dab_fail(ctx, DAB_ERR_ARG, "bad dtype/op");
+    return mapreduce_all_combine(ctx, op, rdt, n, out_host,
+                                 [&](void* slot) { return dab_affine_reduce(ctx, dtype, y, x, a, b, n, op, slot); });
 }
 
 // ---- mailboxes for the fused reduce + combine kernel ---------------------------------------------------------

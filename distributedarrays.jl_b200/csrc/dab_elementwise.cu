@@ -258,13 +258,7 @@ int32_t launch_ew2(dab_ctx* ctx, T* z, const T* x, const T* y, size_t n, F f) {
     return DAB_OK;
 }
 
-// ---- functors --------------------------------------------------------------------------------
-template <typename T>
-struct AffineF {  // a*x + b, two roundings (Julia never contracts; src/broadcast.jl:80 runs Base's loop)
-    T a, b;
-    __device__ __forceinline__ T operator()(T x) const { return jl::add(jl::mul(a, x), b); }
-};
-
+// ---- functors (AffineF, a*x + b, lives in dab_scalar_ops.cuh: the fused broadcast + reduce shares it) ---------------------------
 template <typename T, int FN>
 struct UnaryF {
     __device__ __forceinline__ T operator()(T x) const {

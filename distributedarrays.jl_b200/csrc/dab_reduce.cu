@@ -22,19 +22,34 @@ constexpr int RD_UNROLL = 4;
 
 // Result slot layout (16 bytes at `out`): [0..8) the result in its result dtype, [8..16) the wide accumulator (fp64 for
 // float SUM/PROD -- lets the host see the un-rounded carrier; tests use it).
-template <typename T, typename Map, typename R, typename Out>
-__global__ void __launch_bounds__(RD_THREADS, 8) reduce_kernel(const T* __restrict__ x, size_t n, size_t head, Map map,
+//
+// STORE = true (dab_affine_reduce): the kernel also writes every mapped value to y (evict-first 16-byte stores, before the register
+// tree consumes the pack), so `y .= f.(x); reduce(op, y)` is one pass of 8 instead of 12 bytes per Float32 element.  Grid, tiles,
+// tree and combine are those of the reduce of y, so with x and y at the same offset mod 16 (same head) the result is bit-identical.
+// y may alias x (map!(f, d, d)): each thread loads its packs before it stores them, and neither pointer is declared __restrict__.
+// Resident CTAs per SM the kernel is compiled for: 8 (32 registers) for every plain reduce.  The store variant keeps 8 where it still
+// fits 32 registers without spilling (Float32 SUM / PROD, ptxas -v) and is given 40 registers (6 CTAs per SM) elsewhere.  Occupancy
+// does not change the result; the grid mapping, which decides it, is the same for every instantiation.
+template <typename T, typename R, bool STORE>
+constexpr int rd_min_blocks() {
+    return (!STORE || (sizeof(T) == 4 && (std::is_same<R, SumTraits<T>>::value || std::is_same<R, ProdTraits<T>>::value))) ? 8 : 6;
+}
+
+template <typename T, typename Map, typename R, typename Out, bool STORE = false>
+__global__ void __launch_bounds__(RD_THREADS, rd_min_blocks<T, R, STORE>()) reduce_kernel(const T* x, T* y, size_t n, size_t head, Map map,
                                                              typename R::A* __restrict__ partials, unsigned int* counter,
                                                              void* out, int finalize_mode, long long n_for_all, int tiles_per_cta,
                                                              FusedComm fc) {
     using A = typename R::A;
     using V = typename Map::V;
+    static_assert(!STORE || std::is_same<V, T>::value, "the stored map must keep the element type");
     constexpr int VPT = 16 / sizeof(T);
     __shared__ A smem[RD_THREADS / 32];
     __shared__ bool is_last;
 
     const size_t nvec = (n - head) / VPT;
     const int4* xv = reinterpret_cast<const int4*>(x + head);
+    int4* yv = STORE ? reinterpret_cast<int4*>(y + head) : nullptr;
     constexpr size_t TILE = (size_t)RD_THREADS * RD_UNROLL;
     const size_t ntiles = nvec / TILE;
     A acc = R::identity();
@@ -56,6 +71,12 @@ __global__ void __launch_bounds__(RD_THREADS, 8) reduce_kernel(const T* __restri
             V m[VPT];
 #pragma unroll
             for (int k = 0; k < VPT; ++k) m[k] = map(p.v[k]);
+            if constexpr (STORE) {
+                Pack<T> q;
+#pragma unroll
+                for (int k = 0; k < VPT; ++k) q.v[k] = m[k];
+                st_stream(yv + base + (size_t)u * RD_THREADS, as_int4(q));
+            }
 #pragma unroll
             for (int w = VPT; w > 1; w >>= 1)  // register tree inside one 16-byte vector
 #pragma unroll
@@ -71,13 +92,27 @@ __global__ void __launch_bounds__(RD_THREADS, 8) reduce_kernel(const T* __restri
     if (blockIdx.x == gridDim.x - 1) {  // remainder vectors, unaligned head, tail
         for (size_t i = ntiles * TILE + threadIdx.x; i < nvec; i += RD_THREADS) {
             Pack<T> p = as_pack<T>(ld_stream(xv + i));
-            V m = map(p.v[0]);
+            V mk[VPT];
 #pragma unroll
-            for (int k = 1; k < VPT; ++k) m = R::tile(m, map(p.v[k]));
+            for (int k = 0; k < VPT; ++k) mk[k] = map(p.v[k]);
+            if constexpr (STORE) {
+                Pack<T> q;
+#pragma unroll
+                for (int k = 0; k < VPT; ++k) q.v[k] = mk[k];
+                st_stream(yv + i, as_int4(q));
+            }
+            V m = mk[0];
+#pragma unroll
+            for (int k = 1; k < VPT; ++k) m = R::tile(m, mk[k]);
             acc = R::comb(acc, R::lift(m));
         }
-        for (size_t i = threadIdx.x; i < head; i += RD_THREADS) acc = R::comb(acc, R::lift(map(x[i])));
-        for (size_t i = head + nvec * VPT + threadIdx.x; i < n; i += RD_THREADS) acc = R::comb(acc, R::lift(map(x[i])));
+        auto elem = [&](size_t i) {
+            const V v = map(x[i]);
+            if constexpr (STORE) y[i] = v;
+            acc = R::comb(acc, R::lift(v));
+        };
+        for (size_t i = threadIdx.x; i < head; i += RD_THREADS) elem(i);
+        for (size_t i = head + nvec * VPT + threadIdx.x; i < n; i += RD_THREADS) elem(i);
     }
     acc = block_reduce<R>(acc, smem);
     // ---- two-level "last one out" combine: deterministic, no second launch, tail latency of a few microseconds.
@@ -204,8 +239,8 @@ __global__ void __launch_bounds__(RD_THREADS, 8) reduce_kernel(const T* __restri
     }  // arithmetic Out
 }
 
-template <typename T, typename Map, typename R, typename Out>
-int32_t launch_reduce(dab_ctx* ctx, const T* x, size_t n, Map map, void* out, int finalize_mode) {
+template <typename T, typename Map, typename R, typename Out, bool STORE = false>
+int32_t launch_reduce(dab_ctx* ctx, const T* x, size_t n, Map map, void* out, int finalize_mode, T* y = nullptr) {
     constexpr int VPT = 16 / sizeof(T);
     size_t head = ((16 - ((uintptr_t)x & 15)) & 15) / sizeof(T);
     if (head > n) head = n;
@@ -229,8 +264,8 @@ int32_t launch_reduce(dab_ctx* ctx, const T* x, size_t n, Map map, void* out, in
         fc.nranks = 1;
         fc.op = ctx->fuse_op;
     }
-    reduce_kernel<T, Map, R, Out><<<(unsigned)grid, RD_THREADS, 0, ctx->stream>>>(x, n, head, map, (typename R::A*)ctx->block_partials,
-                                                                                  ctx->counter, out, finalize_mode, (long long)n, (int)k, fc);
+    reduce_kernel<T, Map, R, Out, STORE><<<(unsigned)grid, RD_THREADS, 0, ctx->stream>>>(x, y, n, head, map, (typename R::A*)ctx->block_partials,
+                                                                                         ctx->counter, out, finalize_mode, (long long)n, (int)k, fc);
     DAB_LAUNCHED(ctx);
     return DAB_OK;
 }
@@ -250,6 +285,18 @@ int32_t reduce_arith(dab_ctx* ctx, int32_t op, const T* x, size_t n, void* out) 
             if constexpr (FN == DAB_MAP_ID) return launch_reduce<T, ExtMapF<T>, ExtremaTraits<T>, Pair<T>>(ctx, x, n, ExtMapF<T>{(T)0}, out, 0);
             else return dab_fail(ctx, DAB_ERR_UNSUPPORTED, "extrema with a map is not served (no host fallback)");
         default: return dab_fail(ctx, DAB_ERR_UNSUPPORTED, "reduce op %d needs a predicate map (no host fallback)", op);
+    }
+}
+
+// dab_affine_reduce: the reduce_arith<T, DAB_MAP_ID> switch again, with y .= a.*x .+ b as the map and the stores switched on
+template <typename T>
+int32_t affine_reduce_t(dab_ctx* ctx, int32_t op, T* y, const T* x, size_t n, T a, T b, void* out) {
+    const AffineMap<T> map{AffineF<T>{a, b}};
+    switch (op) {
+        case DAB_SUM: return launch_reduce<T, AffineMap<T>, SumTraits<T>, T, true>(ctx, x, n, map, out, 0, y);
+        case DAB_PROD: return launch_reduce<T, AffineMap<T>, ProdTraits<T>, T, true>(ctx, x, n, map, out, 0, y);
+        case DAB_MAX: return launch_reduce<T, AffineMap<T>, MaxTraits<T>, T, true>(ctx, x, n, map, out, 0, y);
+        default: return launch_reduce<T, AffineMap<T>, MinTraits<T>, T, true>(ctx, x, n, map, out, 0, y);
     }
 }
 
@@ -375,6 +422,28 @@ int32_t dab_reduce(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const v
         case DAB_U8: return reduce_u8(ctx, op, map, (const uint8_t*)x, n, out_dev);
         default: return dab_fail(ctx, DAB_ERR_ARG, "dab_reduce: bad dtype %d", dtype);
     }
+}
+
+// y .= a.*x .+ b, then dab_reduce(op, identity map) of y into out_dev -- in ONE pass when a kernel serves it: Float32 / Float64, op SUM
+// PROD MAX MIN, n > 0, and x and y at the same offset mod 16 (the reduce's head peel, hence its grid, follows the pointer's alignment;
+// only then is the fused result bit-identical to reducing y afterwards).  Any other case runs the two launches it replaces.
+int32_t dab_affine_reduce(dab_ctx* ctx, int32_t dtype, void* y, const void* x, const void* a, const void* b, size_t n, int32_t op,
+                          void* out_dev) {
+    DAB_ENTER(ctx);
+    DAB_REQUIRE(ctx, ((x && y) || n == 0) && a && b, DAB_ERR_ARG, "dab_affine: null pointer");
+    DAB_REQUIRE(ctx, out_dev, DAB_ERR_ARG, "dab_reduce: null pointer");
+    DAB_REQUIRE(ctx, op >= DAB_SUM && op <= DAB_EXTREMA, DAB_ERR_ARG, "dab_reduce: bad op %d", op);
+    const size_t es = dab_dtype_size(dtype);
+    const bool fused = (dtype == DAB_F32 || dtype == DAB_F64) && (op == DAB_SUM || op == DAB_PROD || op == DAB_MAX || op == DAB_MIN) &&
+                       n > 0 && ((uintptr_t)x & 15) == ((uintptr_t)y & 15) && (uintptr_t)x % es == 0;
+    if (!fused) {
+        int32_t st = dab_affine(ctx, dtype, y, x, a, b, n);
+        if (st != DAB_OK) return st;
+        return dab_reduce(ctx, dtype, op, DAB_MAP_ID, nullptr, y, n, out_dev);
+    }
+    if (dtype == DAB_F32)
+        return affine_reduce_t<float>(ctx, op, (float*)y, (const float*)x, n, *(const float*)a, *(const float*)b, out_dev);
+    return affine_reduce_t<double>(ctx, op, (double*)y, (const double*)x, n, *(const double*)a, *(const double*)b, out_dev);
 }
 
 int32_t dab_reduce_host(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const void* map_param, const void* x, size_t n,

@@ -99,6 +99,14 @@ struct MapF {
         else return x;
     }
 };
+// y .= a.*x .+ b fused into the reduction of y (dab_affine_reduce): the mapped value is the broadcast's own AffineF, so the values the
+// kernel stores and reduces are bit for bit what dab_affine writes and the identity-map reduce of y then reads.
+template <typename T>
+struct AffineMap {
+    using V = T;
+    AffineF<T> f;
+    __device__ __forceinline__ V operator()(T x) const { return f(x); }
+};
 template <typename T, int FN>
 struct PredF {
     using V = int;

@@ -103,3 +103,16 @@ __device__ __forceinline__ T sign(T a) {  // Julia sign: keeps +-0 and NaN
 }
 
 }  // namespace jl
+
+namespace {
+
+// y = a*x + b, two roundings (Julia never contracts; src/broadcast.jl:80 runs Base's loop).  The one definition behind the broadcast
+// kernel (dab_elementwise.cu) and the fused broadcast + reduce (AffineMap, dab_reduce.cu): the fused y and its reduction are therefore
+// bit-identical to the broadcast followed by the reduce.
+template <typename T>
+struct AffineF {
+    T a, b;
+    __device__ __forceinline__ T operator()(T x) const { return jl::add(jl::mul(a, x), b); }
+};
+
+}  // namespace

@@ -210,6 +210,11 @@ int32_t dab_reduce(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const v
 /* Same, then copies the 16-byte result slot to out_host and syncs (== remotecall_fetch, src/mapreduce.jl:31). */
 int32_t dab_reduce_host(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const void* map_param, const void* x,
                         size_t n, void* out_host);
+/* y .= a .* x .+ b (dab_affine) followed by dab_reduce(op, DAB_MAP_ID) of y into out_dev, same arguments, same results bit for bit.
+ * Float32 / Float64, op SUM / PROD / MAX / MIN, n > 0 and x, y at the same offset mod 16 (y == x included): ONE kernel reads x, writes
+ * y and reduces the values it has just computed -- 8 instead of 12 bytes per Float32 element.  Any other case runs the two calls. */
+int32_t dab_affine_reduce(dab_ctx* ctx, int32_t dtype, void* y, const void* x, const void* a, const void* b, size_t n, int32_t op,
+                          void* out_dev);
 /* result dtype of dab_reduce for (dtype, op, map). */
 int32_t dab_reduce_result_dtype(int32_t dtype, int32_t op, int32_t map, int32_t* out_dtype);
 /* Caller-side combine  reduce(op, results)  (src/mapreduce.jl:26,34): P < 16 so a plain LEFT FOLD in
@@ -318,6 +323,10 @@ int32_t dab_recv(dab_ctx* ctx, void* recv_dev, size_t nbytes, int32_t peer);
  * fold (dab_combine_ordered) -> host scalar.  Exactly src/mapreduce.jl:29-35. */
 int32_t dab_mapreduce_all(dab_ctx* ctx, int32_t dtype, int32_t op, int32_t map, const void* map_param, const void* x,
                           size_t n, void* out_host);
+/* y .= a .* x .+ b (dab_affine) followed by dab_mapreduce_all(op, DAB_MAP_ID) of y: the chunk reduce is dab_affine_reduce (one
+ * kernel when it fuses), the cross-worker combine is that of dab_mapreduce_all (fused peer combine, or the NCCL all-gather). */
+int32_t dab_affine_mapreduce_all(dab_ctx* ctx, int32_t dtype, void* y, const void* x, const void* a, const void* b, size_t n, int32_t op,
+                                 void* out_host);
 
 /* Fused reduce + combine over NVLink peer memory.  After every rank has created its mailbox (dab_mailbox_create returns the
  * 64-byte CUDA IPC handle), exchanged the handles through the host runtime and attached them (handles = nranks * 64 bytes, in
